@@ -211,6 +211,21 @@ def fill_replay(L, vn, n_fill, rank, distinct_chunks=8, chunk=2048):
         i += n
 
 
+def dump_outputs(out_dir, metrics, batch, params):
+    """Writes what the last timed step hands a caller, one .npy per array: its losses and statistics (float64 scalars,
+    named as b2g_sac_metrics), the per-sample outputs of its minibatch together with the replay slots and policy noise it
+    drew (batch_*, so that identical inputs can be confirmed), and the parameters it left (param_*, '/' written as '__').
+    The step reduces with float atomics, so two runs on identical inputs are not bit-identical: on a B200 (1000 W limit) they
+    agreed to 4e-6 relative after 23 updates, while after 220 updates Adam had grown the differences to the size of the values.
+    Compare builds at a small --warmup + --steps."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.float64(v) for k, v in metrics.items()}
+    arrays.update({"batch_" + k: np.asarray(v, np.float64 if k == "indices" else np.float32) for k, v in batch.items()})
+    arrays.update({"param_" + n.replace("/", "__"): np.asarray(a, np.float32) for n, a in params.items()})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -220,7 +235,7 @@ def main():
     ap.add_argument("--batch", type=int, default=256)
     ap.add_argument("--replay-filled", type=int, default=65536, help="transitions resident in HBM (2 x 32 KiB each: 4 GiB >> 126 MB L2)")
     ap.add_argument("--buffer-size", type=int, default=1_000_000)
-    ap.add_argument("--regions", type=int, default=7, help="timed K-step regions; the MEDIAN region is reported")
+    ap.add_argument("--regions", type=int, default=7, help="the K timed steps are split into this many regions; the MEDIAN region is reported")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--dp", default="p2p", choices=["p2p", "nccl"],
@@ -228,7 +243,13 @@ def main():
     ap.add_argument("--no-c3", action="store_true", help="skip the RGB-D B=1024 extra measurement (config.extra.c3)")
     ap.add_argument("--precision", default="bf16x3", choices=["fp32", "bf16x3", "bf16"],
                     help="bf16x3 = tcgen05 BF16 hi/lo split, the mode that passes the 1e-4 parity tests (default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's losses, per-sample outputs and updated parameters to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -303,23 +324,28 @@ def main():
             parity = {"oracle_batch": B * world, "rel_err": {k: float(f"{v:.3g}") for k, v in errs.items()}, "q1_rel_err_rank0": float(f"{q_err:.3g}"),
                       "tol": 1e-4, "first_step_ok": bool(max(errs.values()) <= 1e-4 and q_err <= 1e-4)}
 
-    # ---- device-resident throughput: R regions of exactly K graph replays each, CUDA events on the learner's stream
-    # (b2g_sac_step brackets the K launches with events), barrier + synchronize on both sides of every region, max over
-    # ranks per region, MEDIAN over regions.  Inputs: random slots of a replay working set far larger than L2.
+    # ---- device-resident throughput: exactly K graph replays, split into R regions of near-equal size, CUDA events on the
+    # learner's stream (b2g_sac_step brackets a region's launches with events), barrier + synchronize on both sides of every
+    # region, max over ranks per region, MEDIAN per-step time over regions.  Inputs: random slots of a replay working set far
+    # larger than L2.
+    n_regions = min(args.regions, args.steps)
+    sizes = [args.steps // n_regions + (i < args.steps % n_regions) for i in range(n_regions)]
     L.step(args.warmup, lr=LR)
     barrier()
     region_ms = []
     with ClockSampler(local) as clk:
         time.sleep(0.25)                       # let the sampler stream before the timed regions start
-        for _ in range(args.regions):
+        for n in sizes:
             barrier()
-            L.step(args.steps, lr=LR)          # one timed region: exactly K steps
+            last = L.step(n, lr=LR)            # one timed region
             region_ms.append(L.last_step_ms())
         barrier()
     region_ms = max_over_ranks(region_ms)
-    ms = float(np.median(region_ms))
-    sync_steps_per_s = args.steps / (ms * 1e-3)
+    ms_step = float(np.median([t / n for t, n in zip(region_ms, sizes)]))
+    sync_steps_per_s = 1e3 / ms_step
     value = world * sync_steps_per_s
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, L.last_batch(), L.get_parameters())
 
     # ---- end to end through the C ABI with pinned HOST batches (H2D of the batch + D2H of the losses per step)
     tr = synth.make_transitions(B, vn["obs_mean"], vn["obs_var"], seed=77 + rank)
@@ -422,7 +448,6 @@ def main():
                        or k.startswith("heads_fc0") or k == "heads_dgrad" or (k == "heads_wgrad" and "fwd_fused" not in prof)}
         gemm_serial = sum(gemm_groups.values())
         share = gemm_serial / sum(prof.values())
-        ms_step = ms / args.steps
         gemm_ms = share * ms_step
         peak_tf, peak_hbm, peak_src = peaks()
         flops = FLOP_PER_STEP_B256 * B / 256
@@ -456,7 +481,7 @@ def main():
             "config": {"workload": WORKLOAD,
                        "global_batch": B * world, "replay_capacity": args.buffer_size, "replay_filled": args.replay_filled,
                        "l2": f"inputs larger than L2: replay working set {args.replay_filled * 2 * 32768 / 2**30:.1f} GiB >> 126 MB; minibatch slots are random per step",
-                       "timing": f"median of {args.regions} regions of {args.steps} steps (CUDA events on the learner's stream, max over ranks per region); regions_ms={[round(x, 3) for x in region_ms]}",
+                       "timing": f"{args.steps} steps in {n_regions} regions of {sizes} steps, median per-step time over regions (CUDA events on the learner's stream, max over ranks per region); regions_ms={[round(x, 3) for x in region_ms]}",
                        "precision": {"fp32": "fp32 FFMA (B2G_PREC_FP32_SIMT)", "bf16x3": "tcgen05 BF16 hi/lo split x3, fp32 TMEM accumulate (B2G_PREC_BF16X3; passes 1e-4 parity)", "bf16": "tcgen05 single-pass BF16 (fast mode, ~5e-4 on Q)"}[args.precision], "parallelism": f"dp{world}" + ("" if world == 1 else (" (gradients reduced, slices updated and parameters broadcast by one kernel over NVLink peer memory)" if args.dp == "p2p" else " (NCCL all-reduce, replicated Adam)")),
                        "sync_steps_per_s": sync_steps_per_s, "numa": numa,
                        "extra": {"c3": c3}},

@@ -4,12 +4,17 @@
   encoder_config.json   its config.yaml (network / encoding_dim) + the last row of history.csv
   golden_encoder.npz    encodings of 8 seeded synthetic depth scenes by the float64 oracle (oracle/encoder_ref.py) and
                         the restated auto-encoder's reconstruction MSE on 64 scenes (the sanity anchor)
+  encoder_model_h5_skeleton.npz
+                        model.h5 with every weight payload cut out (24 KB of HDF5 structure), the offsets the payloads were
+                        cut from and the SHA-256 of the whole file: with encoder_weights.npz it rebuilds model.h5 byte for byte
 
     python tests/golden/make_encoder_fixtures.py
 """
 import csv
+import hashlib
 import json
 import os
+import struct
 import sys
 
 import numpy as np
@@ -28,6 +33,26 @@ OUT = os.path.dirname(os.path.abspath(__file__))
 
 w = h5min.load_keras_weights(os.path.join(SRC, "model.h5"))
 np.savez_compressed(os.path.join(OUT, "encoder_weights.npz"), **{k.replace("/", "__"): v for k, v in w.items()})
+
+raw = open(os.path.join(SRC, "model.h5"), "rb").read()
+cuts = []
+for k, v in w.items():
+    b = np.ascontiguousarray(v, "<f4").tobytes()
+    o = raw.find(b)
+    # the payload occurs once in the file, at an address a layout message names
+    assert o >= 0 and raw.find(b, o + 1) < 0 and struct.pack("<Q", o) in raw, k
+    cuts.append((o, k))
+cuts.sort()
+for (o, k), (nxt, _) in zip(cuts, cuts[1:]):
+    assert o + w[k].nbytes <= nxt, k            # no two payloads overlap
+keep, pos = [], 0
+for o, k in cuts:
+    keep.append(raw[pos:o])
+    pos = o + w[k].nbytes
+keep.append(raw[pos:])
+np.savez_compressed(os.path.join(OUT, "encoder_model_h5_skeleton.npz"), skeleton=np.frombuffer(b"".join(keep), np.uint8),
+                    offsets=np.array([o for o, _ in cuts], np.int64), names=np.array([k for _, k in cuts]),
+                    sha256=hashlib.sha256(raw).hexdigest())
 cfg = yaml.safe_load(open(os.path.join(SRC, "config.yaml")))
 hist = list(csv.DictReader(open(os.path.join(SRC, "history.csv"))))
 json.dump({"network": cfg["network"], "encoding_dim": cfg["encoding_dim"], "alpha": cfg.get("alpha", 0.1),

@@ -1,5 +1,6 @@
 """Perception encoder (SURVEY section 8 row a12), CPU side: the model.h5 reader, the oracle against its committed golden
 encodings, and the reconstruction anchor that ties the restated auto-encoder to the reference's training history."""
+import hashlib
 import json
 import os
 
@@ -12,8 +13,6 @@ from b200grasp import h5min, synth
 from b200grasp.encoders import keras_encoder_arrays
 from oracle import encoder_ref as E
 from tests.util import GOLD
-
-REF_H5 = "/root/reference/encoder_files/new_gripper_encoder/model.h5"
 
 
 def load_fixture():
@@ -32,10 +31,25 @@ def test_fixture_inventory_matches_the_reference_graph():
     assert cfg["encoding_dim"] == 100 and [l["strides"] for l in cfg["network"]] == [2, 2, 2]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_H5), reason="reference tree not present (GPU box)")
-def test_h5_reader_reproduces_the_committed_weights():
+def rebuild_model_h5(w):
+    """The reference's model.h5, byte for byte: its stored HDF5 structure with the committed weights put back where they
+    were cut out (tests/golden/make_encoder_fixtures.py), checked against the SHA-256 of the original file."""
+    sk = np.load(os.path.join(GOLD, "encoder_model_h5_skeleton.npz"))
+    skeleton, raw, s = sk["skeleton"].tobytes(), b"", 0
+    for o, k in zip(sk["offsets"].tolist(), sk["names"].tolist()):
+        n = o - len(raw)                                  # structure bytes in front of this payload
+        raw += skeleton[s:s + n] + np.ascontiguousarray(w[k], "<f4").tobytes()
+        s += n
+    raw += skeleton[s:]
+    assert hashlib.sha256(raw).hexdigest() == str(sk["sha256"])
+    return raw
+
+
+def test_h5_reader_reproduces_the_committed_weights(tmp_path):
     w, _ = load_fixture()
-    got = h5min.load_keras_weights(REF_H5)
+    h5 = tmp_path / "model.h5"
+    h5.write_bytes(rebuild_model_h5(w))
+    got = h5min.load_keras_weights(str(h5))
     assert sorted(got) == sorted(w)
     for k in w:
         assert got[k].dtype == np.float32 and np.array_equal(got[k], w[k]), k
